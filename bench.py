@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — candidate schedules evaluated / second on the SPASE hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path over one batch of synthetic candidates per GPU:
@@ -26,6 +26,11 @@ A "step" is one pass of the hot path over one batch of synthetic candidates per 
            C4 the MILP cannot be built (row count reported) and the GPU plan is held to the area lower bound.
 `configs` = the other BASELINE shapes (C3, C5) as short diagnostic runs; `exchange_check` (N > 1) = the
            peer-memory MIN re-derived with an NCCL all_reduce(MIN) outside the timed region.
+
+--dump-outputs DIR writes what the last timed step returned to its caller (rank 0): DIR/makespan.npy (fp32, one
+per candidate), DIR/candidate_id.npy (fp64, the global id of each of those candidates) and the folded arg-min key
+as DIR/best_makespan.npy (fp32) + DIR/best_candidate_id.npy (fp64).  Inputs are seeded, so two builds run with the
+same arguments can be compared output for output.  Batches above DUMP_CANDIDATES are sampled (fixed seed).
 """
 import argparse
 import json
@@ -49,6 +54,7 @@ WAVE = 148 * 8 * 32           # candidates in one half wave of 32-candidate tile
 B_PER_GPU = WAVE * 28         # 1,060,864 candidates = 14 whole tiles for every resident warp of the persistent
                               # grid (no idle warps in a last partial wave) = 543 MB of encodings per step (> 126 MB L2)
 FALLBACK_HBM_GBS = 6650.0
+DUMP_CANDIDATES = 1 << 22     # at most 48 MB of dumped makespans + ids
 
 
 def bytes_per_candidate(j):
@@ -143,11 +149,12 @@ def _clean_env():
     return env
 
 
-def cpu_arm(steps, warmup, config="C4", timeout=900):
+def cpu_arm(steps, warmup, config="C4", timeout=900, all_steps=False):
     """oracle/cpu_arm.py in its own process (before / without torch): the one CPU measurement both the
-    `cpu_baseline` leg and `--impl reference` report."""
+    `cpu_baseline` leg and `--impl reference` report.  all_steps: time every one of the `steps` steps (no
+    time cap)."""
     cmd = [sys.executable, os.path.join(ROOT, "oracle", "cpu_arm.py"), "--steps", str(steps), "--warmup", str(warmup),
-           "--config", config]
+           "--config", config] + (["--max-seconds", "inf"] if all_steps else [])
     out = subprocess.run(cmd, env=_clean_env(), stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=timeout)
     if out.returncode != 0:
         raise RuntimeError("oracle/cpu_arm.py failed: %s" % out.stderr[-2000:])
@@ -159,7 +166,7 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    r = cpu_arm(args.steps, args.warmup)
+    r = cpu_arm(args.steps, args.warmup, timeout=None, all_steps=True)
     val = r["value"]
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus,
             "steps": r["steps_timed"], "warmup": args.warmup, "ms_per_step": r["ms_per_step_median"],
@@ -171,6 +178,22 @@ def run_reference(args):
                     "ms_per_step_max": r["ms_per_step_max"], "build": r["build"], "cores_how": r["cores_how"]},
             "gpu_launches": 0}
     print(json.dumps(line), flush=True)
+
+
+def dump_outputs(out_dir, out, key, id_base):
+    """The last timed step's outputs as .npy files (see the module docstring)."""
+    from saturn_b200.search import key_makespan
+    mk = out.cpu().numpy()
+    ids = np.arange(mk.shape[0])
+    if mk.shape[0] > DUMP_CANDIDATES:
+        ids = np.sort(np.random.default_rng(0).choice(mk.shape[0], DUMP_CANDIDATES, replace=False))
+    k = int(key.item())
+    arrays = {"makespan": mk[ids].astype(np.float32), "candidate_id": (ids + id_base).astype(np.float64),
+              "best_makespan": np.array([key_makespan(k)], dtype=np.float32),
+              "best_candidate_id": np.array([k & 0xffffffff], dtype=np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class _Task:
@@ -229,7 +252,7 @@ def milp_leg_finish(proc, eng, c4_tasks, c4_plan_makespan, c4_wall):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 200; 5 for --impl reference)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch", type=int, default=B_PER_GPU, help="candidates per GPU per step")
@@ -243,11 +266,19 @@ def main():
     ap.add_argument("--solve-devices", type=int, default=0,
                     help="N = 1 only, opt-in: also time saturn.solver.solve(..., devices=D) — ONE process driving D GPUs "
                          "(it touches GPUs beyond --gpus, so it is never run by default)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's outputs to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
-        if args.steps == 200:
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to --impl ours")
+        if args.steps is None:
             args.steps = 5                                            # default K for the CPU arm: minutes, not hours
         return run_reference(args)
+    if args.steps is None:
+        args.steps = 200
     args.warmup = max(args.warmup, 3)
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -386,6 +417,8 @@ def main():
         all_stats = [rank_stats]
     per_rank = [{"rank": r, "timed_ms": float(x[0]), "kernel_ms_min": float(x[1]), "kernel_ms_median": float(x[2]),
                  "kernel_ms_max": float(x[3]), "kernel_ms_first": float(x[4])} for r, x in enumerate(all_stats)]
+    if args.dump_outputs and rank == 0:                       # before any later leg reuses `out`
+        dump_outputs(args.dump_outputs, out, key, id_base)
 
     # ---- N > 1, outside the timed region: the fused peer-memory MIN against NCCL's
     exchange_check = None

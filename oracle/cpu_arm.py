@@ -14,19 +14,20 @@ What makes the number reproducible:
     CPUs in the affinity mask, capped by the cgroup CPU quota), printed in the result;
   * OMP_PROC_BIND=close, OMP_PLACES=cores, OMP_DYNAMIC=false set before the library is loaded;
   * the C file is compiled on THIS host with -O3 -march=native (-ffp-contract=off kept: results stay
-    bit-identical to the portable -O2 build the parity tests use) into oracle/_native/;
+    bit-identical to the portable -O2 build the parity tests use) into a temporary directory, so that the
+    benchmark writes nothing into the repository tree (which may be read-only);
   * a step is >= 2 M candidate evaluations (a 262 144-candidate sample evaluated repeatedly; the table and
     the sample exceed L2 per core, each candidate is an independent 256-step dependent chain);
   * OpenMP schedule(dynamic) over blocks of candidates; value = median over the timed steps.
 """
 import argparse
 import ctypes
-import hashlib
 import json
 import math
 import os
 import subprocess
 import sys
+import tempfile
 import time
 
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -75,30 +76,18 @@ def physical_cores():
     return n, desc
 
 
-def native_build():
-    """gcc -O3 -march=native of oracle/ref_eval.c for this host -> oracle/_native/libref_eval_<tag>.so"""
+def native_build(out_dir):
+    """gcc -O3 -march=native of oracle/ref_eval.c for this host -> out_dir/libref_eval_native.so"""
     src = os.path.join(HERE, "ref_eval.c")
-    try:
-        with open("/proc/cpuinfo") as f:
-            info = [ln for ln in f if ln.startswith(("model name", "flags"))][:2]
-    except OSError:
-        info = []
-    with open(src, "rb") as f:
-        tag = hashlib.sha1(("".join(info)).encode() + f.read()).hexdigest()[:12]
-    out_dir = os.path.join(HERE, "_native")
-    so = os.path.join(out_dir, "libref_eval_%s.so" % tag)
+    so = os.path.join(out_dir, "libref_eval_native.so")
     flags = ["-O3", "-march=native", "-fopenmp", "-shared", "-fPIC", "-ffp-contract=off"]
-    if not os.path.exists(so):
-        os.makedirs(out_dir, exist_ok=True)
-        tmp = so + ".%d.tmp" % os.getpid()
-        try:
-            subprocess.check_call(["gcc"] + flags + [src, "-o", tmp, "-lm"])
-            os.replace(tmp, so)
-        except (OSError, subprocess.CalledProcessError):
-            # no compiler on this host: fall back to the portable build shipped with the snapshot
-            sys.path.insert(0, ROOT)
-            from oracle import c_oracle
-            return c_oracle.build(), "gcc -O2 (portable build; native compile failed)"
+    try:
+        subprocess.check_call(["gcc"] + flags + [src, "-o", so, "-lm"])
+    except (OSError, subprocess.CalledProcessError):
+        # no compiler on this host: fall back to the portable oracle/libref_eval.so the package build made
+        sys.path.insert(0, ROOT)
+        from oracle import c_oracle
+        return c_oracle.build(), "gcc -O2 (portable build; native compile failed)"
     return so, "gcc " + " ".join(flags[:2])
 
 
@@ -122,8 +111,9 @@ def main():
     os.environ["OMP_DYNAMIC"] = "false"
     os.environ.setdefault("OMP_WAIT_POLICY", "active")
 
-    so, build = native_build()
-    lib = ctypes.CDLL(so)
+    with tempfile.TemporaryDirectory(prefix="saturn_b200_cpu_arm_") as tmp:
+        so, build = native_build(tmp)
+        lib = ctypes.CDLL(so)                         # stays mapped after the directory is removed
     fn = lib.ref_eval_f32
     fn.restype = ctypes.c_int
     fn.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int,

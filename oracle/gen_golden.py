@@ -294,7 +294,34 @@ def main_rerun(fname, name):
     raise SystemExit("no such case")
 
 
+def main_layout():
+    """The reference's `saturn` package as data: every module file and the top-level functions it defines.
+    tests/test_host_logic.py rebuilds an empty-bodied stand-in distribution from it to check the alias
+    package's fall-through without the reference installed."""
+    import ast
+    modules, functions = [], {}
+    for dirpath, dirnames, files in os.walk(os.path.join(REF, "saturn")):
+        dirnames.sort()
+        for f in sorted(files):
+            if f.endswith(".py"):
+                path = os.path.join(dirpath, f)
+                rel = os.path.relpath(path, REF)
+                modules.append(rel)
+                with open(path) as fh:
+                    names = [n.name for n in ast.parse(fh.read()).body if isinstance(n, ast.FunctionDef)]
+                if names:
+                    functions[rel] = names
+    out = {"generator": "oracle/gen_golden.py --layout", "reference_commit": "b65e3d2", "modules": modules,
+           "functions": functions}
+    dst = os.path.join(os.path.dirname(HERE), "tests", "golden", "reference_layout.json")
+    with open(dst, "w") as f:
+        json.dump(out, f, indent=1)
+    print("wrote", dst, len(modules), "modules")
+
+
 def main():
+    if "--layout" in sys.argv:
+        return main_layout()
     if "--rerun" in sys.argv:
         i = sys.argv.index("--rerun")
         return main_rerun(sys.argv[i + 1], sys.argv[i + 2])

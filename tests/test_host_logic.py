@@ -259,11 +259,22 @@ def test_forecast_matches_reference_forecast():
 
 
 # ------------------------------------------------------------------------------------------ round 2
-def test_alias_package_falls_through_to_an_installed_reference():
+def test_alias_package_falls_through_to_an_installed_reference(tmp_path):
     """`import saturn` is this repository's alias; submodules it does not implement resolve in a reference
-    distribution when one is on sys.path (saturn_b200/_alias.py) and raise a clear ImportError otherwise."""
+    distribution when one is on sys.path (saturn_b200/_alias.py) and raise a clear ImportError otherwise.
+    The reference is a stand-in with the reference package's module layout (tests/golden/reference_layout.json):
+    every module file exists and each top-level function returns the path of the file that defines it."""
+    import json
     import subprocess
     import sys
+    with open(os.path.join(ROOT, "tests", "golden", "reference_layout.json")) as f:
+        layout = json.load(f)
+    ref = tmp_path / "reference"
+    for rel in layout["modules"]:
+        path = ref / rel
+        path.parent.mkdir(parents=True, exist_ok=True)
+        path.write_text("".join("def %s(*args, **kwargs):\n    return %r\n" % (name, rel)
+                                for name in layout["functions"].get(rel, [])))
     code = r'''
 import sys
 sys.path.insert(0, %r)
@@ -280,19 +291,19 @@ try:
     raise SystemExit("saturn.executor.execute must not resolve without a reference distribution")
 except ImportError as e:
     assert "not part of the B200 solver drop-in" in str(e)
-ref = "/root/reference"
-import os
-if os.path.isdir(ref):
-    sys.path.append(ref)
-    for m in [m for m in sys.modules if m == "saturn" or m.startswith("saturn.")]:
-        del sys.modules[m]
-    import saturn, saturn.solver, saturn.library
-    assert saturn.library.__file__.startswith(ref)                      # fell through
-    assert saturn.solver.solve.__module__ == "saturn_b200.solver"       # the drop-in still wins
-    assert saturn.orchestrate.__module__ == "saturn_b200.orchestrator"
+ref = %r
+sys.path.append(ref)
+for m in [m for m in sys.modules if m == "saturn" or m.startswith("saturn.")]:
+    del sys.modules[m]
+import saturn, saturn.solver, saturn.library, saturn.core.representations as Rp, saturn.executor as E
+assert saturn.library.__file__.startswith(ref)                      # fell through
+assert saturn.solver.solve.__module__ == "saturn_b200.solver"       # the drop-in still wins
+assert saturn.orchestrate.__module__ == "saturn_b200.orchestrator"
+assert E.execute() == "saturn/executor/executor.py"                 # names the drop-in lacks come from the reference
+assert Rp.search() == "saturn/core/representations/Strategy.py"
 print("ok")
-''' % ROOT
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd="/tmp")
+''' % (ROOT, str(ref))
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd=str(tmp_path))
     assert r.returncode == 0 and r.stdout.strip().endswith("ok"), r.stdout + r.stderr
 
 
